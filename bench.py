@@ -318,7 +318,7 @@ def _oracle_port(workload):
 
 def cpu_steady_windows(workload, h, w, budget_s, max_windows, cores):
     """Time steady-state windows of the reference's CPU forward at LR h x w on `cores` host threads.  Uses the UNMODIFIED
-    reference (oracle/ref_loader.py: /root/reference or the staged copy oracle/_ref/RefVSR) through its public API
+    reference (oracle/ref_loader.py: the copy staged under oracle/_ref/RefVSR) through its public API
     SRNet.forward, with the propagated state primed instead of computed (a first window costs minutes; the steady
     window's cost does not depend on the state's values) -> kind 'reference'.  Falls back to the oracle port
     (kind 'port') only when no reference checkout exists.  Returns (kind, [seconds per window])."""
@@ -489,6 +489,7 @@ def clip_leg(args, net, dev, world, rank, wl):
 
 
 def run_ours(args):
+    import numpy as np
     import torch
     import torch.distributed as dist
     from refvsr_b200.dist import exchange_halo, plan_segments
@@ -630,24 +631,31 @@ def run_ours(args):
         n0 = net.Network.executed_kernels
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        fn(Wm, Wm + K)
+        last = fn(Wm, Wm + K)
         e1.record()
         barrier()
         clocks = sampler.stop()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item()), net.Network.executed_kernels - n0, clocks
+        return float(ms.item()), net.Network.executed_kernels - n0, clocks, last
 
     # one-time CUDA-graph capture (one graph per ring phase x window kind, ~16 of them) in an untimed pre-pass over
     # the same windows, so that the K timed steps measure the steady serving rate rather than capture cost
     net.Network.reset_state()
     run_resident(0, Wm + K)
-    ms_res, launches, clocks = timed(run_resident)
-    ms_e2e, _, clocks_e2e = timed(run_e2e)
+    dump = args.dump_outputs if rank == 0 else None
+    ms_res, launches, clocks, last = timed(run_resident)
+    # the engine reuses its output buffer on the next call: copy the last timed step's result out now
+    result = last['result'].float().cpu() if dump else None
+    ms_e2e, _, clocks_e2e, _ = timed(run_e2e)
     bad = {'hw_slowdown', 'hw_thermal_slowdown', 'sw_thermal_slowdown'}
     if bad & set(clocks['reasons']):                          # re-measure once (timing rules)
-        ms_res, launches, clocks = timed(run_resident)
+        ms_res, launches, clocks, last = timed(run_resident)
+        result = last['result'].float().cpu() if dump else None
+    if dump:
+        os.makedirs(dump, exist_ok=True)
+        np.save(os.path.join(dump, 'result.npy'), result.numpy())
 
     # sustained leg (N = 1): >= 5 s of consecutive windows of one long stream, with its own clock record - MEASURED_PEAKS shows
     # this GPU settling well below its 1965 MHz boost under seconds-long dense load, which a 0.2 s timed region never sees
@@ -797,7 +805,11 @@ def main():
     ap.add_argument('--sustained-s', type=float, default=5.0)
     ap.add_argument('--no-graphs', action='store_true', help='eager kernel launches (for ncu launch lists)')
     ap.add_argument('--fuse', action='store_true', help='use the fused residual-block kernel (rv_resblock)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write forward()['result'] of the last timed step (rank 0) to DIR/result.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3) if args.impl == 'ours' else args.warmup
     if args.impl == 'reference':
         run_reference(args)

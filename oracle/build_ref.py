@@ -46,9 +46,7 @@ def build(src=SRC, dst=DST, verbose=True):
 
 
 def ref_root():
-    """path of a usable reference checkout: /root/reference here, the staged copy on the GPU box; None if neither"""
-    if os.path.isfile(os.path.join(SRC, 'models', 'SRNet.py')):
-        return SRC
+    """path of the staged reference copy (what build() made), None when nothing is staged"""
     if os.path.isfile(os.path.join(DST, 'models', 'SRNet.py')):
         return DST
     return None

@@ -1,8 +1,8 @@
 """TEST / BENCH INFRASTRUCTURE - imports the UNMODIFIED reference (codeslake/RefVSR) as a Python package tree.
 
-Source: /root/reference in the build container, else the byte-for-byte staged copy oracle/_ref/RefVSR (oracle/build_ref.py)
-on the GPU box.  Third-party packages the reference imports but this image lacks (mmcv, easydict, termcolor) come from
-oracle/shims.  Only tests/, bench.py's reference / eager_b200 / cpu_baseline legs and __graft_entry__.smoke() may use this.
+Source: the byte-for-byte copy build() stages under oracle/_ref/RefVSR (oracle/build_ref.py).  Third-party packages
+the reference imports but this image lacks (mmcv, easydict, termcolor) come from oracle/shims.  Only tests/, bench.py's
+reference / eager_b200 / cpu_baseline legs and __graft_entry__.smoke() may use this.
 """
 import importlib
 import os
@@ -48,7 +48,7 @@ def build_reference(config_name, device='cpu', seed=1234, **overrides):
     from refvsr_b200.modules import seeded_test_weights
     cls = reference_srnet_class()
     if cls is None:
-        raise RuntimeError('no reference checkout: neither /root/reference nor oracle/_ref/RefVSR (python oracle/build_ref.py)')
+        raise RuntimeError('no reference copy staged under oracle/_ref/RefVSR (python oracle/build_ref.py)')
     cfg = importlib.import_module('configs.' + config_name).get_config('p', 'm', config_name)
     is_cuda = str(device).startswith('cuda')
     cfg.cuda, cfg.device, cfg.dist = is_cuda, ('cuda' if is_cuda else 'cpu'), False      # run.py:399-405

@@ -86,9 +86,41 @@ def build_case(name, spec, RefSRNet):
     print(name, 'written', os.path.getsize(path) // 1024, 'KiB')
 
 
+# tests/test_oracle_golden.py::test_oracle_matches_live_reference: a shape / seed outside CASES.  A full result per window
+# would make a large file, so a seeded sample of each result is stored, with its mean and mean square.
+LIVE = dict(config='config_RefVSR_small_MFID', over=dict(num_blocks=2), T=5, h=28, w=36, ref_scale=1, frames=3, seed=77)
+LIVE_NAME, LIVE_SAMPLES = 'live_small_mfid_t5_28x36', 4096
+
+
+def build_live(RefSRNet):
+    from refvsr_b200.modules import seeded_test_weights
+    from refvsr_b200.synth import make_clip, sliding_windows
+    spec = LIVE
+    cfg = importlib.import_module('configs.' + spec['config']).get_config('p', 'm', spec['config'])
+    cfg.cuda, cfg.device, cfg.dist = False, 'cpu', False
+    for k, v in spec['over'].items():
+        setattr(cfg, k, v)
+    ref = RefSRNet(cfg).eval()
+    seeded_test_weights(ref, seed=spec['seed'])
+    lrs, refs = make_clip(spec['frames'], spec['h'], spec['w'], spec['ref_scale'], seed=spec['seed'])
+    n = 3 * 16 * spec['h'] * spec['w']
+    out = {'sample_idx': np.sort(np.random.default_rng(spec['seed']).choice(n, LIVE_SAMPLES, replace=False)).astype(np.int32)}
+    with torch.no_grad():
+        for k, wl, wr, first in sliding_windows(lrs, refs, spec['T']):
+            res = ref(wl, wr, first, False, False)['result'][0].double().flatten()
+            out[f'sample_{k}'] = res[torch.from_numpy(out['sample_idx']).long()].numpy().astype(np.float32)
+            out[f'moments_{k}'] = np.array([float(res.mean()), float((res * res).mean())])
+    out['meta'] = np.array([spec['T'], spec['h'], spec['w'], spec['ref_scale'], spec['frames'], spec['seed']])
+    path = os.path.join(ROOT, 'tests', 'golden', LIVE_NAME + '.npz')
+    np.savez_compressed(path, **out)
+    print(LIVE_NAME, 'written', os.path.getsize(path) // 1024, 'KiB')
+
+
 if __name__ == '__main__':
     RefSRNet = load_reference()
     for name, spec in CASES.items():
         if len(sys.argv) > 1 and name not in sys.argv[1:]:
             continue
         build_case(name, spec, RefSRNet)
+    if len(sys.argv) == 1 or LIVE_NAME in sys.argv[1:]:
+        build_live(RefSRNet)

@@ -9,7 +9,7 @@ PYTHONPATH (INTEGRATION.md section 1, verbatim) - and the per-frame PSNR / SSIM 
     the data_loader drop-in, is_first handling across two videos.
   * GPU (-m gpu): the real CUDA path under DataParallel, the ptflops init forward, and autocast, against the unmodified
     reference in eager PyTorch on the same GPU (staged copy oracle/_ref/RefVSR).  Bar: |dPSNR| < 0.01 dB (north_star).
-The reference checkout is /root/reference when present, else the staged copy (oracle/build_ref.py)."""
+The reference checkout is the copy build() stages under oracle/_ref (oracle/build_ref.py); without one these tests skip."""
 import os
 import re
 import subprocess

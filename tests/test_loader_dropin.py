@@ -1,6 +1,6 @@
 """Drop-in `data_loader` (decoded-frame cache): the reference's own Test_datasets returns bit-identical items with
-and without it, and decodes each file once per stream instead of T times.  Needs the reference checkout (build
-container only) - the GPU box has no /root/reference, where this test skips."""
+and without it, and decodes each file once per stream instead of T times.  Needs the reference copy that build()
+stages under oracle/_ref (oracle/build_ref.py); skips where none is staged."""
 import json
 import os
 import subprocess
@@ -8,14 +8,17 @@ import sys
 
 import pytest
 
+from oracle.build_ref import ref_root
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REF = ref_root()
 
 CODE = r'''
 import sys, os, json, hashlib, time
 import numpy as np
 from PIL import Image
-root, tmp, use_dropin = sys.argv[1], sys.argv[2], sys.argv[3] == '1'
-sys.path[:0] = ([os.path.join(root, 'refvsr_b200', 'dropin')] if use_dropin else []) + [os.path.join(root, 'oracle', 'shims'), '/root/reference', root]
+root, tmp, use_dropin, ref_root = sys.argv[1], sys.argv[2], sys.argv[3] == '1', sys.argv[4]
+sys.path[:0] = ([os.path.join(root, 'refvsr_b200', 'dropin')] if use_dropin else []) + [os.path.join(root, 'oracle', 'shims'), ref_root, root]
 import importlib
 cfg = importlib.import_module('configs.config_RefVSR_small_MFID').get_config('p', 'm', 'config_RefVSR_small_MFID')
 cfg.dist = False
@@ -59,16 +62,16 @@ def _make_clip(tmp):
                 Image.fromarray(rng.integers(0, 256, (h, w, 3), dtype=np.uint8)).save(os.path.join(d, f'{k:04d}.png'))
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/data_loader'), reason='reference checkout not present on this box')
+@pytest.mark.skipif(REF is None, reason='no reference copy staged under oracle/_ref')
 def test_cached_loader_returns_identical_items(tmp_path):
     _make_clip(str(tmp_path))
     out = {}
     for flag in ('0', '1'):
-        r = subprocess.run([sys.executable, '-c', CODE, ROOT, str(tmp_path), flag], capture_output=True, text=True, timeout=600)
+        r = subprocess.run([sys.executable, '-c', CODE, ROOT, str(tmp_path), flag, REF], capture_output=True, text=True, timeout=600)
         assert r.returncode == 0, r.stderr[-3000:]
         out[flag] = json.loads(r.stdout.strip().splitlines()[-1])
     ref, ours = out['0'], out['1']
-    assert '/root/reference' in ref['utils_file'] and 'dropin' in ours['utils_file']
+    assert ref['utils_file'].startswith(REF) and 'dropin' in ours['utils_file']
     assert ours['items'] == ref['items'] == 10
     assert ours['meta'] == ref['meta']
     assert ours['sha'] == ref['sha'], 'every tensor of every item must be bit-identical'
