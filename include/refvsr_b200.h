@@ -166,6 +166,22 @@ typedef struct {
 } rv_conv_chain_desc;
 int rv_conv_chain(const rv_conv_chain_desc* d, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * rv_dcn3x3 - modulated deformable 3x3 convolution (DCNv2), the ModulatedDCNPack of the RefVSR_IR refill extractor
+ * (models/archs/edvr_net.py:15-58: conv_offset -> chunk / cat / sigmoid -> mmcv modulated_deform_conv2d with stride 1,
+ * pad 1, dilation 1, groups 1, 8 deform groups), minus conv_offset itself, which is an ordinary rv_conv2d:
+ *   om (H, W, om_cs) fp32, om_cs >= 216: conv_offset's RAW output.  For deform group g (input channels 8g..8g+7) and
+ *      tap k = 3*ky + kx:  dy = om[18g + 2k], dx = om[18g + 2k + 1], m = sigmoid(om[144 + 9g + k]);
+ *   x  (H, W, 64) `dtype`, 16-byte aligned;
+ *   s  = bilinear(x[.., c], y - 1 + ky + dy, x - 1 + kx + dx): 0 when the sample lies at or beyond one pixel outside the
+ *        map (h <= -1, h >= H, w <= -1, w >= W), corners outside the map contribute 0 (mmcv dmcn_im2col_bilinear);
+ *   out[(y, x)][n] = act(bias[n] + sum_{k, c} W[n][c][ky][kx] * m * s),  n < cout <= 64, out (H, W, out_cs) `dtype`.
+ * impl RV_CONV_IMPL_TC: tcgen05 implicit GEMM, f16 / bf16, wpack = packing.pack_tc(W, [(64, 64)], dtype, nb, layout=1);
+ * impl RV_CONV_IMPL_SIMT: CUDA cores, any dtype, wpack = packing.pack_simt(W, [(64, 64)]) fp32 (nb ignored).
+ * ------------------------------------------------------------------------------------------------ */
+int rv_dcn3x3(const void* x, const float* om, int om_cs, int H, int W, int dtype, const void* wpack, const float* bias,
+              int cout, int nb, int act, int impl, void* out, int out_cs, void* stream);
+
 /* space-to-depth by 2: out[(Y,X)][(ry*2+rx)*C + c] = src[(2Y+ry, 2X+rx)][c].  Turns the two stride-2
  * convolutions of the path (ref_encoder2.0.0, RefVSR.py:45; aa2.align.p_conv.0, alignment.py:21) into
  * stride-1 3x3 convolutions over 4C channels (weights re-indexed by packing.s2d_weights), so they run on

@@ -68,6 +68,7 @@ SIGNATURES = {
     'rv_conv2d_tc_plan': (_I, [C.POINTER(rv_conv_desc), _I, _I, C.POINTER(C.c_int32)]),
     'rv_resblock': (_I, [C.POINTER(rv_resblock_desc), _P]),
     'rv_conv_chain': (_I, [C.POINTER(rv_conv_chain_desc), _P]),
+    'rv_dcn3x3': (_I, [_P, _P, _I, _I, _I, _I, _P, _P, _I, _I, _I, _I, _P, _I, _P]),
     'rv_space_to_depth2': (_I, [_P, _I, _I, _I, _I, _P, _P]),
     'rv_prep_image': (_I, [_P, _I, _I, _P, _I, _P, _I, _I, _P]),
     'rv_spynet_resize_norm': (_I, [_P, _I, _I, _P, _I, _I, _P]),
@@ -219,6 +220,20 @@ class CudaOps:
             d.nbuf, d.H, d.W, d.C, d.dtype, d.nb = len(bufs), H, W, Cc, DTYPE_CODE[bufs[0].dtype], nb
             d.layers, d.nlayers, d.flags, d.max_ctas = arr, len(part), flags.data_ptr(), int(max_ctas)
             _check(self.lib, self.lib.rv_conv_chain(C.byref(d), self._stream()), 'rv_conv_chain')
+
+    def dcn3x3(self, layer, x, om, out, act=ACT_NONE):
+        """modulated deformable 3x3 conv (rv_dcn3x3): `layer` = packing.pack_dcn(...), x (H, W, 64), om (H, W, >= 216) fp32 raw
+        conv_offset output, out (H, W, >= cout) in x's dtype"""
+        assert (layer.kh, layer.kw, layer.alloc0, layer.alloc1) == (3, 3, 64, 0), f'{layer.name}: not a 64-channel 3x3 DCN'
+        assert layer.impl != IMPL_TC or layer.layout == 1, f'{layer.name}: the tensor-core DCN reads the layout-1 image ([9][nb][64])'
+        _chk_dev(x, om, out)
+        H, W, Cc = x.shape
+        assert Cc == 64, f'{layer.name}: x has {Cc} channels, the DCN reads 64'
+        assert om.dtype == torch.float32 and tuple(om.shape[:2]) == (H, W) and tuple(out.shape[:2]) == (H, W)
+        assert out.dtype == x.dtype
+        _check(self.lib, self.lib.rv_dcn3x3(_ptr(x), _ptr(om), om.shape[2], H, W, DTYPE_CODE[x.dtype], _ptr(layer.wpack),
+                                            _ptr(layer.bias), layer.cout, layer.nb, act, layer.impl, _ptr(out), out.shape[2],
+                                            self._stream()), f'rv_dcn3x3[{layer.name}]')
 
     def space_to_depth2(self, src, out):
         _chk_dev(src, out)

@@ -257,6 +257,13 @@ def pack_conv_uncached(name, weight, bias, srcs, stride, pad, act_dtype, device,
                       kh * kw * (alloc0 + alloc1), wp, b.to(device).contiguous())
 
 
+def pack_dcn(name, weight, bias, act_dtype, device):
+    """weight (cout <= 64, 64, 3, 3) of a ModulatedDCNPack -> the operand rv_dcn3x3 reads: the single-box tensor-core image
+    ([9 taps][nb][64], layout 1) for 16-bit activations, fp32 [576][ceil4(cout)] for the CUDA-core variant"""
+    assert weight.shape[1:] == (64, 3, 3) and weight.shape[0] <= 64, f'{name}: {tuple(weight.shape)} is not a 64-channel 3x3 DCN'
+    return pack_conv(name, weight, bias, [(64, 64)], 1, 1, act_dtype, device, tc_layout=1)
+
+
 @dataclass
 class PackedResBlock:
     name: str
